@@ -5,6 +5,7 @@
     torchrun --nproc-per-node N ... bench.py --gpus N ...          # one rank per GPU (driver launches this)
     python bench.py --impl reference --gpus 1 --steps 20 --warmup 5  # the UNMODIFIED reference on the host cores
     python bench.py --batch 4096 --dim 768                         # another BASELINE.json config (configs[1])
+    python bench.py --dump-outputs DIR                             # also write the last timed step's outputs (.npy)
 
 Workload (BASELINE.json `metric`): per-rank batch B=16384, D=1024, bf16, W = --gpus text chunks per rank,
 synthetic L2-normalised features (seed 1234 + rank), t' = log 10, b = -10. One "step" = one forward + backward of the
@@ -165,6 +166,31 @@ def synth(rank: int, B: int, D: int):
     img = torch.nn.functional.normalize(torch.randn(B, D, generator=g))
     txt = torch.nn.functional.normalize(torch.randn(B, D, generator=g))
     return img.to(torch.bfloat16), txt.to(torch.bfloat16)
+
+
+DUMP_NAMES = ("loss", "dimg", "dtxt", "dt_prime", "dbias")
+DUMP_GRAD_ELEMENTS = 7 << 20       # per gradient: two float32 samples of 28 MiB keep a dump under 64 MB
+
+
+def dump_outputs(out_dir: str, outputs):
+    """Writes one step's (loss, dimg, dtxt, dt', dbias) as <out_dir>/<name>.npy: float64 where the step returned
+    float64, float32 otherwise. Gradients of more than DUMP_GRAD_ELEMENTS elements are cut to a fixed, seeded sample of
+    rows (the same rows for both); grad_rows.npy lists the row indices."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = dict(zip(DUMP_NAMES, outputs))
+    B, D = arrays["dimg"].shape
+    rows = torch.arange(B)
+    if B * D > DUMP_GRAD_ELEMENTS:
+        rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:DUMP_GRAD_ELEMENTS // D].sort().values
+    for name in ("dimg", "dtxt"):
+        arrays[name] = arrays[name][rows.to(arrays[name].device)]
+    arrays["grad_rows"] = rows
+    for name, t in arrays.items():
+        wide = t.dtype in (torch.float64, torch.int64)
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().to(torch.float64 if wide else torch.float32).numpy())
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -418,6 +444,7 @@ def run_ours(args):
     bt = torch.tensor([-10.0], device=dev)
     img_d, txt_d = img.detach(), txt.detach()
 
+    # every variant of a step returns what its caller receives: (loss, dimg, dtxt, dt', dbias)
     if args.api == "module":
         def step():
             img.grad = None
@@ -426,10 +453,10 @@ def run_ours(args):
             mod.bias.grad = None
             loss = mod(img, txt)
             loss.backward()
-            return loss
+            return loss, img.grad, txt.grad, mod.t_prime.grad, mod.bias.grad
     elif args.api == "fused":   # the fused C-ABI entry siglip_fwd_bwd (BASELINE.json configs[1] "fused fwd+bwd"), bf16 gradients
         def step():
-            return eng.fwd_bwd(img_d, txt_d, tpt, bt, torch.bfloat16)[0]
+            return eng.fwd_bwd(img_d, txt_d, tpt, bt, torch.bfloat16)
     else:   # the same fused C-ABI step captured once into a CUDA graph and replayed (single rank only: the cross-rank
             # flag values of a multi-rank step are kernel parameters that advance every step)
         if world > 1:
@@ -447,7 +474,7 @@ def run_ours(args):
 
         def step():
             graph.replay()
-            return graph_out[0]
+            return graph_out
 
     def barrier():
         if world > 1:
@@ -502,11 +529,16 @@ def run_ours(args):
     barrier()
     first_sample = sampler.mark()
     e0.record()
-    for _ in range(args.steps):
-        loss = step()
+    for _ in range(args.steps - 1):
+        step()                  # outputs held until the next step returns would double its buffers (a cudaMalloc)
+    outputs = step()
     e1.record()
     barrier()
     last_sample = sampler.mark()
+    loss = outputs[0]
+    # copies: later replays of the graph overwrite its output buffers
+    dumped = [t.detach().clone() for t in outputs] if (args.dump_outputs and rank == 0) else None
+    del outputs
     nvl1 = _nvlink_counters(local_rank) if (rank == 0 and world > 1) else None
     my_clock = sampler.median_since(first_sample)
     ms_mine = e0.elapsed_time(e1)
@@ -766,6 +798,8 @@ def run_ours(args):
             except Exception as ex:  # noqa: BLE001
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": None, "kind": "reference",
                                         "sample": f"failed: {ex}"}
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -797,7 +831,15 @@ def main():
     ap.add_argument("--clock-period-ms", type=float, default=5.0, help="NVML clock / throttle-reason sampling period")
     ap.add_argument("--sustain-ms", type=float, default=600.0,
                     help="minimum GPU time of the warm-up (power-capped sustained clocks at every N)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them returned on rank 0 (loss, dimg, dtxt, "
+                         "dt_prime, dbias) as DIR/<name>.npy, at most 64 MB: larger gradients are cut to a seeded "
+                         "sample of rows, listed in grad_rows.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's path, not of --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

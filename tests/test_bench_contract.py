@@ -49,10 +49,54 @@ def test_reference_arm_extrapolates_at_n_gt_1():
     assert "extrapolated" in d["cpu_baseline"]["sample"]
 
 
+def _bench_module():
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_steps_must_be_positive():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                         text=True, timeout=60, cwd=ROOT)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
+@pytest.mark.parametrize("B,D", [(48, 40), (16384, 1024)])
+def test_dump_outputs_files(tmp_path, B, D):
+    """What --dump-outputs writes for one step's outputs: float32 / float64 .npy files, at most 64 MB in all; a gradient
+    too large for that is cut to the same seeded rows in every run."""
+    import numpy as np
+    import torch
+
+    bench = _bench_module()
+    g = torch.Generator().manual_seed(5)
+    outputs = (torch.tensor(9.25), torch.randn(B, D, generator=g).to(torch.bfloat16),
+               torch.randn(B, D, generator=g).to(torch.bfloat16), torch.tensor(-0.5, dtype=torch.float64),
+               torch.tensor(0.75))
+    bench.dump_outputs(str(tmp_path / "a"), outputs)
+    bench.dump_outputs(str(tmp_path / "b"), outputs)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(n + ".npy" for n in bench.DUMP_NAMES + ("grad_rows",))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in names) <= 64e6
+    z = {f[:-4]: np.load(tmp_path / "a" / f) for f in names}
+    assert all(v.dtype in (np.float32, np.float64) for v in z.values())
+    assert z["dt_prime"].dtype == np.float64 and z["loss"].dtype == np.float32
+    assert float(z["loss"]) == 9.25 and float(z["dt_prime"]) == -0.5 and float(z["dbias"]) == 0.75
+    rows = z["grad_rows"].astype(np.int64)
+    assert len(rows) == min(B, bench.DUMP_GRAD_ELEMENTS // D) and np.all(np.diff(rows) > 0)
+    for i, name in ((1, "dimg"), (2, "dtxt")):
+        assert np.array_equal(z[name], outputs[i].float().numpy()[rows])
+    for f in names:
+        assert np.array_equal(np.load(tmp_path / "b" / f), z[f[:-4]])
+
+
 @pytest.mark.gpu
-def test_product_arm_line():
+def test_product_arm_line(tmp_path):
     d = _run(["--gpus", "1", "--steps", "3", "--warmup", "3", "--batch", "2048", "--dim", "256", "--sustain-ms", "50",
-              "--cpu-steps", "1"])
+              "--cpu-steps", "1", "--dump-outputs", str(tmp_path)])
     assert "impl" not in d and BASE_KEYS | {"gpu_launches", "clocks", "roofline", "cpu_baseline", "burst", "parity",
                                             "per_rank"} <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 3 and d["warmup"] >= 3 and d["dtype"] == "bf16"
@@ -69,3 +113,17 @@ def test_product_arm_line():
     par = d["parity"]
     assert par["pass"] is True and par["shape"] == [2048, 768]
     assert all(v <= 1e-3 for v in par["fused_fp32"].values())
+    # --dump-outputs: the last timed step's module outputs (bf16 gradients), against fp32 autograd on the bench inputs
+    import numpy as np
+
+    bench = _bench_module()
+    z = {n: np.load(tmp_path / (n + ".npy")) for n in bench.DUMP_NAMES + ("grad_rows",)}
+    assert float(z["loss"]) == d["loss"]
+    assert z["dimg"].shape == z["dtxt"].shape == (2048, 256) and np.array_equal(z["grad_rows"], np.arange(2048))
+    img, txt = bench.synth(0, 2048, 256)
+    loss, dimg, dtxt, dtp, db = bench._fp32_autograd(img, [txt], np.log(10.0), -10.0, 0)
+    dtxt = dtxt[0]
+    assert abs(float(z["loss"]) - loss) <= 1e-3 * abs(loss)
+    assert abs(float(z["dt_prime"]) - dtp) <= 1e-3 * abs(dtp) and abs(float(z["dbias"]) - db) <= 1e-3 * abs(db)
+    for got, ref in ((z["dimg"], dimg), (z["dtxt"], dtxt)):
+        assert np.linalg.norm(got - ref.numpy()) <= 4e-3 * np.linalg.norm(ref.numpy())

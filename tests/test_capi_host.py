@@ -113,32 +113,47 @@ def test_chunk_schedule_covers_every_pair_once(world, bidir):
         assert chunk_schedule(0, world, True)[1:3] == [1, world - 1]
 
 
-def test_reference_copy_for_the_cpu_arm_is_byte_identical():
-    """tools/fetch_ref.py places the unmodified reference under the git-ignored baseline/_ref; where /root/reference is
-    present (build container) every copied file must have the upstream bytes, and the manifest must say so."""
+def test_reference_copy_for_the_cpu_arm_is_byte_identical(tmp_path, monkeypatch):
+    """tools/fetch_ref.py copies the unmodified reference verbatim under the git-ignored baseline/_ref and writes the
+    sha256 of every file into a manifest. The recipe is checked on a stand-in source tree; a copy that build() placed
+    in this tree must carry the upstream digests pinned in tests/golden/reference_sha256.json."""
     import hashlib
     import json
+    import shutil
 
-    src = "/root/reference"
-    dst = os.path.join(ROOT, "baseline", "_ref")
-    if not os.path.isdir(src):
-        pytest.skip("the reference tree is only present in the build container")
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     try:
         import fetch_ref
-        assert fetch_ref.fetch(src, quiet=True)
     finally:
         sys.path.pop(0)
-    manifest = json.load(open(os.path.join(dst, "MANIFEST.json")))["sha256"]
-    assert "distributed_sigmoid_loss.py" in manifest and "rwightman_sigmoid_loss.py" in manifest
+    src, dst = tmp_path / "src", tmp_path / "dst"
+    src.mkdir()
+    for i, name in enumerate(fetch_ref.FILES):
+        (src / name).write_bytes(f"# {name}\n".encode() + bytes(range(256)) * (i + 1))
+    monkeypatch.setattr(fetch_ref, "DEST", str(dst))
+    assert fetch_ref.fetch(str(src), quiet=True)
+    manifest = json.load(open(dst / "MANIFEST.json"))["sha256"]
+    assert sorted(manifest) == sorted(fetch_ref.FILES)
     for name, digest in manifest.items():
-        a = open(os.path.join(src, name), "rb").read()
-        b = open(os.path.join(dst, name), "rb").read()
+        a, b = (src / name).read_bytes(), (dst / name).read_bytes()
         assert a == b and hashlib.sha256(b).hexdigest() == digest, name
-    # the directory stays out of the history
-    out = subprocess.run(["git", "check-ignore", "baseline/_ref/distributed_sigmoid_loss.py"], cwd=ROOT,
+
+    pinned = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_sha256.json")))["sha256"]
+    assert sorted(pinned) == sorted(fetch_ref.FILES)
+    copy = os.path.join(ROOT, "baseline", "_ref")
+    if os.path.exists(os.path.join(copy, "MANIFEST.json")):
+        assert json.load(open(os.path.join(copy, "MANIFEST.json")))["sha256"] == pinned
+        for name, digest in pinned.items():
+            assert hashlib.sha256(open(os.path.join(copy, name), "rb").read()).hexdigest() == digest, name
+
+    # the directory stays out of the history (checked against the .gitignore alone: a checkout need not be a clone)
+    repo = tmp_path / "repo"
+    repo.mkdir()
+    shutil.copyfile(os.path.join(ROOT, ".gitignore"), repo / ".gitignore")
+    subprocess.run(["git", "init", "-q"], cwd=repo, check=True)
+    out = subprocess.run(["git", "check-ignore", "baseline/_ref/distributed_sigmoid_loss.py"], cwd=repo,
                          capture_output=True, text=True)
-    assert out.returncode == 0
+    assert out.returncode == 0, out.stderr
 
 
 def test_bench_parity_reference_agrees_with_the_pinned_oracle():
